@@ -9,6 +9,7 @@ so the worst case is what is timed; nothing is skipped).
 
   python bench.py --gpus N --steps K --warmup W            (ours; torchrun for N > 1)
   python bench.py --impl reference ...                     (the CPU restatement on host cores)
+  python bench.py ... --dump-outputs DIR                   (also saves the last timed step's tokens: DIR/tokens.npy)
 
 `value`  device-resident inputs, timed with CUDA events per step (L2 flushed between steps),
          max over ranks, whole-job aggregate over N GPUs (weak scaling: 64 segments per GPU).
@@ -298,6 +299,13 @@ def run_ours(args):
     launches = _lib.launch_count() - launches0
     total_ms = sum(a.elapsed_time(b) for a, b in evs)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # the legs below reuse `tokens`: take the last timed step's ids now, every rank's segments in global order
+        dump = mt3_dist.gather_tokens(tokens.clone(), world * B).cpu().numpy()
+        if rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "tokens.npy"), dump.astype(np.float32))   # ids < 2^24: exact
+            log(f"wrote {args.dump_outputs}/tokens.npy {dump.shape}")
 
     log(f"timed {args.steps} steps: {total_ms / args.steps:.1f} ms/step; e2e leg")
     # ---- e2e: public API with HOST buffers (H2D + D2H inside the timed region) ----------------
@@ -605,7 +613,14 @@ def main():
                     help="encoder/cross-K/V GEMMs: exact fp32 CUDA cores, or tcgen05 tf32 (x3 = fp32-faithful split)")
     ap.add_argument("--workload", default="batch", choices=["batch", "longform"],
                     help="batch: BASELINE configs[1]/[2] (64 segments per GPU, the headline); longform: configs[4] (3 min of audio, strong scaling)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="batch workload: write the raw token ids of the last timed step, all segments of all GPUs, "
+                         "to DIR/tokens.npy (float32 [segments, 1024], 0 past --dec-steps)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "batch"):
+        ap.error("--dump-outputs needs --impl ours --workload batch")
     if args.impl == "reference":
         return run_reference(args)
     if args.workload == "longform":

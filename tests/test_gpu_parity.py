@@ -823,3 +823,24 @@ def test_tensor_core_encoder_parity(mode, tol, attn, monkeypatch):
     e_l = np.abs(lg - logits64).max() / np.abs(logits64).max()
     print(f"logits[{mode}]: gpu vs fp64 {e_l:.3e}")
     assert e_l <= (LOGIT_TOL if tol is None else tol)
+
+
+def test_bench_dump_outputs_are_the_timed_paths_tokens(tmp_path):
+    """`bench.py --dump-outputs DIR` saves the token ids of its last timed step: bench's seeded 64-segment batch through
+    the same pass via InferenceModel gives them again, bit for bit."""
+    import subprocess
+    import sys
+    import bench
+    from mt3_b200 import inference
+    steps = 8
+    cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--dec-steps", str(steps),
+           "--no-alt-kv", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)]
+    out = subprocess.run(cmd, capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    got = np.load(tmp_path / "tokens.npy")
+    assert got.dtype == np.float32 and got.shape == (bench.BATCH_PER_GPU, 1024)
+    assert (got[:, steps:] == 0).all() and (got[:, :steps] > 0).any()
+    im = inference.InferenceModel('synthetic:0', 'mt3', device=DEV, batch_size=bench.BATCH_PER_GPU)
+    want = im.transcribe_segments(bench.synth_audio(bench.BATCH_PER_GPU, 1234), num_steps=steps, stop_at_eos=False,
+                                  decoded=False)
+    np.testing.assert_array_equal(got, want.astype(np.float32))

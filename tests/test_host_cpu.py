@@ -272,6 +272,9 @@ def test_bench_reference_arm_contract():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     other = subprocess.run(cmd[:2] + ["--impl", "reference", "--gpus", "2"], capture_output=True, text=True, timeout=120, cwd=root, env=env)
     assert other.returncode == 0 and other.stdout.strip() == ""
+    for bad in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "d"], ["--workload", "longform", "--dump-outputs", "d"]):
+        rejected = subprocess.run(cmd[:2] + bad, capture_output=True, text=True, timeout=120, cwd=root)
+        assert rejected.returncode == 2 and rejected.stdout == "" and bad[-2] in rejected.stderr, bad
 
 
 @pytest.mark.parametrize("top_level_target", [False, True])
@@ -350,57 +353,46 @@ def test_program_granularities():
             assert (len(mapped) == 0 and name == 'flat') or mapped[0] == prog(g.program_map_fn(p))
 
 
-# ---- against the reference checkout itself (build container only: /root/reference does not travel to the GPU box) ----
-REF = "/root/reference/mt3"
-needs_reference = pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present")
-
-
-@needs_reference
+# ---- against what the reference's own files give (stored by tests/golden/make_golden.py) ----------------------------
 def test_gin_lite_reads_the_references_own_gin_files():
     """The reference's gin files, unmodified, give the same model surface as the package's copies (gin/model.gin:47-59,
-    gin/mt3.gin, gin/ismir2021.gin) -- and InferenceModel(gin_dir=<reference>/gin) is how a user points at them."""
+    gin/mt3.gin, gin/ismir2021.gin); gin_reference.json holds what gin_lite read from the reference's files."""
     from mt3_b200 import gin_lite
+    gold = json.load(open(os.path.join(GOLD, "gin_reference.json")))
     bindings = ['VOCAB_CONFIG=@vocabularies.VocabularyConfig()', 'vocabularies.VocabularyConfig.num_velocity_bins=%NUM_VELOCITY_BINS']
     for mt in ("mt3", "ismir2021"):
         ours = gin_lite.parse_config_files_and_bindings([os.path.join(ROOT, "mt3_b200", "gin", f) for f in ("model.gin", mt + ".gin")], bindings)
-        ref = gin_lite.parse_config_files_and_bindings([os.path.join(REF, "gin", f) for f in ("model.gin", mt + ".gin")], bindings)
-        po, pr = ours.params('network.T5Config'), ref.params('network.T5Config')
+        ref = gold[mt]
+        po, pr = ours.params('network.T5Config'), ref["T5Config"]
         for k in ('emb_dim', 'num_heads', 'head_dim', 'mlp_dim', 'num_encoder_layers', 'num_decoder_layers', 'dropout_rate',
                   'logits_via_embedding'):
             assert po[k] == pr[k], k
         assert tuple(po['mlp_activations']) == tuple(pr['mlp_activations'])
-        assert ours.macro('TASK_FEATURE_LENGTHS') == ref.macro('TASK_FEATURE_LENGTHS')
-        assert (ours.binding('vocabularies.VocabularyConfig', 'num_velocity_bins')
-                == ref.binding('vocabularies.VocabularyConfig', 'num_velocity_bins'))
+        assert ours.macro('TASK_FEATURE_LENGTHS') == ref["TASK_FEATURE_LENGTHS"]
+        assert ours.binding('vocabularies.VocabularyConfig', 'num_velocity_bins') == ref["num_velocity_bins"]
 
 
-@needs_reference
 def test_event_codec_equals_the_references_module_on_random_events():
-    """mt3/event_codec.py is the one reference module that imports with the standard library alone: loaded by path, it and
-    mt3_b200.event_codec agree on every index of the mt3 and ismir2021 codecs, on the event type ranges and on the errors."""
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("ref_event_codec", os.path.join(REF, "event_codec.py"))
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
+    """mt3/event_codec.py is the one reference module that imports with the standard library alone: mt3_b200.event_codec
+    and the tables it produced (event_codec_tables.json) agree on every index of the mt3 and ismir2021 codecs, on the
+    event type ranges and on the errors."""
     from mt3_b200 import event_codec as ours, vocabularies as V
+    gold = json.load(open(os.path.join(GOLD, "event_codec_tables.json")))
     for nvb in (1, 127):
         co = V.build_codec(V.VocabularyConfig(num_velocity_bins=nvb))
-        cr = ref.Codec(max_shift_steps=co.max_shift_steps, steps_per_second=co.steps_per_second,        # vocabularies.py:119-140
-                       event_ranges=[ref.EventRange('pitch', 0, 127), ref.EventRange('velocity', 0, nvb), ref.EventRange('tie', 0, 0),
-                                     ref.EventRange('program', 0, 127), ref.EventRange('drum', 0, 127)])
-        assert co.num_classes == cr.num_classes
+        cr = gold[str(nvb)]
+        assert co.num_classes == cr["num_classes"] == len(cr["events"])
         for i in range(co.num_classes):
-            eo, er = co.decode_event_index(i), cr.decode_event_index(i)
-            assert (eo.type, eo.value) == (er.type, er.value)
-            assert co.encode_event(ours.Event(eo.type, eo.value)) == cr.encode_event(ref.Event(er.type, er.value)) == i
-            assert co.is_shift_event_index(i) == cr.is_shift_event_index(i)
+            eo, er = co.decode_event_index(i), cr["events"][i]
+            assert [eo.type, eo.value] == er
+            assert co.encode_event(ours.Event(eo.type, eo.value)) == i
+            assert co.is_shift_event_index(i) == bool(cr["is_shift"][i])
         for t in ('shift', 'pitch', 'velocity', 'tie', 'program', 'drum'):
-            assert tuple(co.event_type_range(t)) == tuple(cr.event_type_range(t))
-        for bad in (ours.Event('pitch', 128), ours.Event('nope', 0)):
+            assert list(co.event_type_range(t)) == cr["ranges"][t]
+        assert [['pitch', 128], ['nope', 0]] == cr["encode_raises"]
+        for t, v in cr["encode_raises"]:
             with pytest.raises(ValueError):
-                co.encode_event(bad)
-            with pytest.raises(ValueError):
-                cr.encode_event(ref.Event(bad.type, bad.value))
-        for c in (co, cr):
-            with pytest.raises(ValueError):
-                c.decode_event_index(co.num_classes)
+                co.encode_event(ours.Event(t, v))
+        assert cr["decode_raises"] == [co.num_classes]
+        with pytest.raises(ValueError):
+            co.decode_event_index(co.num_classes)
