@@ -6,8 +6,9 @@
 //
 //  sgemm_dec_cluster_kernel   exact-fp32 GEMM for M <= 64 rows, the default.  One thread-block CLUSTER (8 CTAs; 16 for
 //                      the long-K MLP-out projection) per 64 x 32 output tile splits K; 4 x 4 register tiles, packed FFMA2.
-//                      Every CTA pushes the rows owned by rank r into rank r's shared memory and, after one cluster
-//                      barrier, each rank sums its rows in rank order (deterministic) and runs the fused epilogue:
+//                      Every CTA pushes the rows owned by rank r into rank r's shared memory (by default one bulk
+//                      DSMEM copy per peer onto the peer's mbarrier, operand loads staged under the multiply:
+//                      MT3_DEC_PIPE) and each rank sums its rows in rank order (deterministic) and runs the fused epilogue:
 //                      RMSNorm factor (statistic computed from the A tiles the GEMM loads anyway, layers.py:613-616),
 //                      residual, gated GELU, head-major KV-cache append (fp32 or fp16 cache), per-tile sums of squares
 //                      of the output.  (A second warp group per CTA splitting the K chunk once more is written in the
@@ -250,7 +251,8 @@ sgemm_dec_kernel(const DecGemmArgs p) {
 // rank r into rank r's shared memory (st.shared::cluster); after ONE cluster barrier every rank sums the S partials
 // of its own rows from LOCAL shared memory in rank order (bit-reproducible), applies the fused epilogue and stores.
 // No global scratch, no atomics, no second barrier (nobody reads remote memory after the barrier, so a CTA may exit
-// as soon as it is done).
+// as soon as it is done).  The default (MT3_DEC_PIPE=3, below) stages the loads under the multiply and replaces the
+// stores + barrier by bulk copies that complete on each receiver's own mbarrier.
 //
 // Arithmetic: exact fp32 FMA, k ascending inside a group, as packed FFMA2 (ffma2() in common.cuh).  The tensor-core
 // variants of round 1 (mma.sync 3xTF32, tcgen05 3xTF32) were parity-green but not faster and live in
@@ -267,12 +269,47 @@ __device__ __forceinline__ void st_cluster_f4(uint32_t addr, float4 v) {
 __device__ __forceinline__ void st_cluster_f1(uint32_t addr, float x) {
   asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(addr), "f"(x) : "memory");
 }
+// local shared memory -> a peer's shared memory (DSMEM) by the bulk-copy engine; completion is counted in bytes on the
+// peer's mbarrier (dst and bar: shared::cluster addresses of the same CTA)
+__device__ __forceinline__ void bulk_s2c(uint32_t dst, uint32_t src, uint32_t bytes, uint32_t bar) {
+  asm volatile("cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+               ::"r"(dst), "r"(src), "r"(bytes), "r"(bar) : "memory");
+}
+// wait for the bytes sent to this CTA (phase 0 of its exchange mbarrier); cluster-scope acquire: the writers are peers.
+// Bounded spin like tc::mbar_wait.
+__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
+  uint32_t ok = 0, spins = 0;
+  do {
+    asm volatile(
+        "{\n\t.reg .pred P;\n\t"
+        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 P, [%1], %2;\n\t"
+        "selp.b32 %0, 1, 0, P;\n\t}"
+        : "=r"(ok)
+        : "r"(tc::smem_u32(bar)), "r"(parity)
+        : "memory");
+    if (!ok && ++spins > (1u << 26)) __trap();
+  } while (!ok);
+}
+// cp.async.wait_group takes an immediate: n = groups that may still be pending (0 .. 7)
+__device__ __forceinline__ void cp_async_wait_pending(int n) {
+  switch (n) {
+    case 0: asm volatile("cp.async.wait_group 0;" ::: "memory"); break;
+    case 1: asm volatile("cp.async.wait_group 1;" ::: "memory"); break;
+    case 2: asm volatile("cp.async.wait_group 2;" ::: "memory"); break;
+    case 3: asm volatile("cp.async.wait_group 3;" ::: "memory"); break;
+    case 4: asm volatile("cp.async.wait_group 4;" ::: "memory"); break;
+    case 5: asm volatile("cp.async.wait_group 5;" ::: "memory"); break;
+    case 6: asm volatile("cp.async.wait_group 6;" ::: "memory"); break;
+    default: asm volatile("cp.async.wait_group 7;" ::: "memory"); break;
+  }
+}
 
 constexpr int kDecLDB = kDecBN + 8;            // padded weight rows
 constexpr int kDecRedFloats = 8 * 8 * kDecBN;  // [src rank][local rows][32 cols] partials pushed to this CTA (S*R = 64 rows)
-template <int KC, int G>
+template <int KC, int G, int PIPE>
 constexpr size_t dec_cluster_smem() {
-  return (size_t)(kDecBM * (KC + 4) + KC * kDecLDB + kDecRedFloats + 64 + (G > 1 ? kDecBM * kDecBN : 0)) * sizeof(float);
+  return (size_t)(kDecBM * (KC + 4) + KC * kDecLDB + kDecRedFloats + 64 + (G > 1 ? kDecBM * kDecBN : 0)) * sizeof(float) +
+         ((PIPE & 2) ? 16 : 0);   // exchange mbarrier
 }
 
 // Sum this rank's 64/S rows over the S source ranks (rank order, local shared memory) and apply the fused epilogue:
@@ -328,18 +365,35 @@ __device__ __forceinline__ void dec_reduce_epilogue(const DecGemmArgs& p, const 
   }
 }
 
-template <int KC, bool TRACE, int S, int G>
+// PIPE (MT3_DEC_PIPE, bitmask; 0 = the plain sequence above).  Neither bit changes an FMA, its operands or its order:
+//  bit 0, staged loads: the activations arrive in cp.async groups of kDecStageK k-steps (one trip of the multiply loop);
+//         the multiply of stage s waits for stage s only, so the FMAs start while later stages are still in flight.
+//         The weights are issued before the PDL wait as in the plain form and travel in the first group.
+//  bit 1, bulk exchange: each CTA writes its partial tile (and per-row sums of squares) row-major into its own, now dead,
+//         activation buffer and sends rank r's rows with ONE cp.async.bulk shared::cta -> shared::cluster copy per peer,
+//         completing on the receiver's mbarrier; a rank reduces as soon as ITS bytes have landed -- no second cluster
+//         barrier, so ranks no longer wait for the slowest peer to finish receiving.
+// Measured on a B200 (1000 W limit), whole 64-segment batch, one process (profiles/r03_call1_ab_dec_pipe.txt): 0 454.6,
+// 1 432.4, 2 442.6, 3 429.7 ms -- both bits win, and together most; 3 is the default.
+constexpr int kDecStageK = 16;
+
+template <int KC, bool TRACE, int S, int G, int PIPE>
 __device__ __forceinline__ void dec_cluster_body(const DecGemmArgs& p, const int tile_x) {
   constexpr int BM = kDecBM, BN = kDecBN, NT = 128 * G, LDA = KC + 4, LDB = kDecLDB;
   constexpr int R = BM / S;                   // rows of the tile each rank owns (8 for clusters of 8, 4 for clusters of 16)
   constexpr int KG = KC / G;                  // k-steps per warp group
   static_assert(KG % 4 == 0 && (KC / (2 * G)) % 4 == 0, "K chunk must split into float4 pieces per group / per ssq thread");
+  constexpr bool STAGED = (PIPE & 1) != 0, BULK = (PIPE & 2) != 0;
+  constexpr int NS = KC / kDecStageK;         // load stages
+  static_assert(!STAGED || (G == 1 && KC % kDecStageK == 0 && NS <= 8), "staged loads: one warp group, K chunk of 16 k-step stages");
+  static_assert(!BULK || BM * (BN + 1) <= BM * LDA, "bulk exchange: the partial tile + sums of squares are staged in the activation buffer");
   extern __shared__ __align__(16) float dsm[];
   float* As = dsm;                            // [BM][LDA] activations, row-major
   float* Bs = As + BM * LDA;                  // [KC][LDB] weights
   float* Red = Bs + KC * LDB;                 // [S src][R rows][BN] partial tiles of MY rows (written by all ranks)
   float* Rss = Red + kDecRedFloats;           // [S src][R rows] partial sums of squares of my rows
   float* Part = Rss + 64;                     // [BM][BN] partial tile of warp group 1 (G == 2)
+  uint64_t* xbar = reinterpret_cast<uint64_t*>(Part + (G > 1 ? BM * BN : 0));   // exchange mbarrier (bulk exchange)
 
   unsigned rank;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
@@ -359,12 +413,20 @@ __device__ __forceinline__ void dec_cluster_body(const DecGemmArgs& p, const int
       if (blockIdx.y < 8) p.trace[8 + blockIdx.y] = smid;
     }
   }
+  // bulk exchange: the mbarrier the peers' copies complete on, armed for all S * (R rows + R sums of squares) words
+  // before the cluster arrive below, which publishes it (fence.mbarrier_init) to the peers
+  if constexpr (BULK) {
+    if (tid == 0) {
+      tc::mbar_init(xbar, 1);
+      tc::mbar_arrive_expect_tx(xbar, (uint32_t)(S * R * (BN + 1) * 4));
+      tc::fence_barrier_init();
+    }
+  }
   // "I am running": peers may write into my shared memory once every CTA of the cluster has arrived here
   asm volatile("barrier.cluster.arrive.relaxed.aligned;" ::: "memory");
 
-  // ---- load phase: cp.async (global -> shared, no register staging): all of the CTA's weights and activations
-  // are in flight at once; one wait.  Weights are issued BEFORE the PDL wait (they do not depend on the
-  // previous kernel).
+  // ---- load phase: cp.async (global -> shared, no register staging).  Weights are issued BEFORE the PDL wait (they
+  // do not depend on the previous kernel).
   for (int idx = tid; idx < KC * 8; idx += NT) {
     const int kr = idx >> 3, nq = idx & 7;
     const bool ok = n0 + nq * 4 < p.N;
@@ -374,32 +436,54 @@ __device__ __forceinline__ void dec_cluster_body(const DecGemmArgs& p, const int
   }
   pdl_wait();
   pdl_trigger();
-  for (int idx = tid; idx < KC * 16; idx += NT) {
-    const int row = idx / (KC / 4), kq = idx % (KC / 4);
-    const bool ok = row < p.M;
-    const int col = kbeg + kq * 4;
-    const float* src = (p.A2 != nullptr && col >= p.K0) ? p.A2 + (long long)(ok ? row : 0) * p.lda2 + (col - p.K0)
-                                                         : p.A + (long long)(ok ? row : 0) * p.lda + col;
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(tc::smem_u32(&As[row * LDA + kq * 4])), "l"(src),
-                 "r"(ok ? 16 : 0) : "memory");
+  if constexpr (STAGED) {
+    // activations in NS commit groups of kDecStageK k-steps (64 rows x 4 float4 each); the multiply waits stage by stage
+#pragma unroll
+    for (int s = 0; s < NS; ++s) {
+      for (int idx = tid; idx < BM * (kDecStageK / 4); idx += NT) {
+        const int row = idx / (kDecStageK / 4), kq = s * (kDecStageK / 4) + idx % (kDecStageK / 4);
+        const bool ok = row < p.M;
+        const int col = kbeg + kq * 4;
+        const float* src = (p.A2 != nullptr && col >= p.K0) ? p.A2 + (long long)(ok ? row : 0) * p.lda2 + (col - p.K0)
+                                                             : p.A + (long long)(ok ? row : 0) * p.lda + col;
+        asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(tc::smem_u32(&As[row * LDA + kq * 4])), "l"(src),
+                     "r"(ok ? 16 : 0) : "memory");
+      }
+      asm volatile("cp.async.commit_group;" ::: "memory");
+    }
+  } else {
+    // all of the CTA's activations in flight at once; one wait
+    for (int idx = tid; idx < KC * 16; idx += NT) {
+      const int row = idx / (KC / 4), kq = idx % (KC / 4);
+      const bool ok = row < p.M;
+      const int col = kbeg + kq * 4;
+      const float* src = (p.A2 != nullptr && col >= p.K0) ? p.A2 + (long long)(ok ? row : 0) * p.lda2 + (col - p.K0)
+                                                           : p.A + (long long)(ok ? row : 0) * p.lda + col;
+      asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(tc::smem_u32(&As[row * LDA + kq * 4])), "l"(src),
+                   "r"(ok ? 16 : 0) : "memory");
+    }
+    asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory");
+    __syncthreads();
+    if (tr0) p.trace[2] = (unsigned long long)(clock64() - c0);    // loads landed
   }
-  asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory");
-  __syncthreads();
-  if (tr0) p.trace[2] = (unsigned long long)(clock64() - c0);      // loads landed
 
   // sum of squares of this CTA's K chunk: 2 G threads per row, each a contiguous piece, fixed butterfly order
+  // (staged loads: once the last stage has landed)
   float ss = 0.f;
-  if (p.norm) {
-    constexpr int PIECE = KC / (2 * G);
-    const float* ar = As + (tid / (2 * G)) * LDA + (tid % (2 * G)) * PIECE;
+  auto sum_squares = [&]() {
+    if (p.norm) {
+      constexpr int PIECE = KC / (2 * G);
+      const float* ar = As + (tid / (2 * G)) * LDA + (tid % (2 * G)) * PIECE;
 #pragma unroll
-    for (int k = 0; k < PIECE; k += 4) {
-      const float4 v = *reinterpret_cast<const float4*>(ar + k);
-      ss = fmaf(v.x, v.x, ss); ss = fmaf(v.y, v.y, ss); ss = fmaf(v.z, v.z, ss); ss = fmaf(v.w, v.w, ss);
+      for (int k = 0; k < PIECE; k += 4) {
+        const float4 v = *reinterpret_cast<const float4*>(ar + k);
+        ss = fmaf(v.x, v.x, ss); ss = fmaf(v.y, v.y, ss); ss = fmaf(v.z, v.z, ss); ss = fmaf(v.w, v.w, ss);
+      }
+      ss += __shfl_xor_sync(0xffffffffu, ss, 1);
+      if (G == 2) ss += __shfl_xor_sync(0xffffffffu, ss, 2);
     }
-    ss += __shfl_xor_sync(0xffffffffu, ss, 1);
-    if (G == 2) ss += __shfl_xor_sync(0xffffffffu, ss, 2);
-  }
+  };
+  if constexpr (!STAGED) sum_squares();
 
   // ---- multiply: thread tile rows ty + 16 i (i < 4), columns tx*4 .. +3 (two float2 accumulators per row); warp
   // group g covers k in [g KG, (g+1) KG), ascending ----
@@ -410,8 +494,7 @@ __device__ __forceinline__ void dec_cluster_body(const DecGemmArgs& p, const int
   {
     const float* Ag = As + grp * KG;
     const float* Bg = Bs + grp * KG * LDB;
-#pragma unroll 4
-    for (int k = 0; k < KG; k += 4) {
+    auto fma4 = [&](int k) {                                        // k-steps k .. k+3
       float4 a[4], b[4];
 #pragma unroll
       for (int i = 0; i < 4; ++i) a[i] = *reinterpret_cast<const float4*>(&Ag[(ty + 16 * i) * LDA + k]);
@@ -426,6 +509,20 @@ __device__ __forceinline__ void dec_cluster_body(const DecGemmArgs& p, const int
           ffma2(acc[i][1], av[kk], make_float2(b[kk].z, b[kk].w));
         }
       }
+    };
+    if constexpr (STAGED) {
+#pragma unroll 1
+      for (int s = 0; s < NS; ++s) {                                // one trip per stage, k ascending as below
+        cp_async_wait_pending(NS - 1 - s);
+        __syncthreads();                                            // rows of As are filled by other threads
+        if (tr0 && s == 0) p.trace[2] = (unsigned long long)(clock64() - c0);   // first stage landed
+#pragma unroll
+        for (int k = s * kDecStageK; k < (s + 1) * kDecStageK; k += 4) fma4(k);
+      }
+      sum_squares();
+    } else {
+#pragma unroll 4
+      for (int k = 0; k < KG; k += 4) fma4(k);
     }
   }
   if (G == 2) {                                                     // group 1 -> shared memory -> added by group 0
@@ -448,116 +545,159 @@ __device__ __forceinline__ void dec_cluster_body(const DecGemmArgs& p, const int
 
   const uint32_t red_base = tc::smem_u32(Red) + rank * (R * BN * 4);     // my slot [rank][..] in the owner's Red
   const uint32_t rss_base = tc::smem_u32(Rss) + rank * (R * 4);
-  if (grp == 0) {
+  if constexpr (BULK) {
+    // partial tile [BM][BN] row-major, then the BM row sums of squares, over the activation buffer: rank r's rows are
+    // one contiguous R * BN * 4-byte slice
+    float* Xs = As;
+    __syncthreads();                                                // every read of As (multiply, sums of squares) is done
+    if (grp == 0) {
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {                                  // row ty + 16 i -> owner rank, local row
-      const int row = ty + 16 * i;
-      st_cluster_f4(cluster_map(red_base + (uint32_t)(((row % R) * BN + tx * 4) * 4), (unsigned)(row / R)),
-                    make_float4(acc[i][0].x, acc[i][0].y, acc[i][1].x, acc[i][1].y));
+      for (int i = 0; i < 4; ++i)
+        *reinterpret_cast<float4*>(&Xs[(ty + 16 * i) * BN + tx * 4]) = make_float4(acc[i][0].x, acc[i][0].y, acc[i][1].x, acc[i][1].y);
     }
+    if ((tid % (2 * G)) == 0) Xs[BM * BN + tid / (2 * G)] = ss;
+    tc::fence_proxy_async();                                        // generic-proxy stores -> the bulk copies read them
+    __syncthreads();
+    if (tid < S) {                                                  // thread r sends rank r its rows
+      const uint32_t bar = cluster_map(tc::smem_u32(xbar), (unsigned)tid);
+      bulk_s2c(cluster_map(red_base, (unsigned)tid), tc::smem_u32(Xs + tid * R * BN), (uint32_t)(R * BN * 4), bar);
+      bulk_s2c(cluster_map(rss_base, (unsigned)tid), tc::smem_u32(Xs + BM * BN + tid * R), (uint32_t)(R * 4), bar);
+      asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+    }
+    if (grp == 0) mbar_wait_cluster(xbar, 0);                       // my rows from all S ranks have landed
+  } else {
+    if (grp == 0) {
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {                                // row ty + 16 i -> owner rank, local row
+        const int row = ty + 16 * i;
+        st_cluster_f4(cluster_map(red_base + (uint32_t)(((row % R) * BN + tx * 4) * 4), (unsigned)(row / R)),
+                      make_float4(acc[i][0].x, acc[i][0].y, acc[i][1].x, acc[i][1].y));
+      }
+    }
+    if (p.norm && (tid % (2 * G)) == 0) {
+      const int row = tid / (2 * G);
+      st_cluster_f1(cluster_map(rss_base + (uint32_t)((row % R) * 4), (unsigned)(row / R)), ss);
+    }
+    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
   }
-  if (p.norm && (tid % (2 * G)) == 0) {
-    const int row = tid / (2 * G);
-    st_cluster_f1(cluster_map(rss_base + (uint32_t)((row % R) * 4), (unsigned)(row / R)), ss);
-  }
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
   if (tr0) p.trace[4] = (unsigned long long)(clock64() - c0);      // partials exchanged
 
   if (grp == 0) dec_reduce_epilogue<S>(p, Red, Rss, rank, n0);
+  // the CTA (and its staging buffer) must outlive the bulk copies' reads of it
+  if (BULK && tid < S) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
   if (tr) {
     if (tr0) p.trace[5] = (unsigned long long)(clock64() - c0);    // reduce + epilogue stores issued
     atomicMax(p.trace + 1, gtime_ns());
   }
 }
 
-template <int KC, bool TRACE, int S, int G>
+template <int KC, bool TRACE, int S, int G, int PIPE>
 __global__ void __launch_bounds__(128 * G)
 sgemm_dec_cluster_kernel(const DecGemmArgs p) {
-  dec_cluster_body<KC, TRACE, S, G>(p, (int)blockIdx.x);
+  dec_cluster_body<KC, TRACE, S, G, PIPE>(p, (int)blockIdx.x);
 }
 
 // Two independent GEMMs that read the same inputs in ONE launch (column tiles [0, tiles0) belong to p0, the rest to
 // p1): used for  y' = y + o.Wo  together with  q_raw = [o | y].[Wo.Wq ; Wq]  (the out-projection folded into the
 // next projection with a precomposed weight block), which removes a kernel from the dependency chain.
-template <int KC0, int KC1, bool TRACE, int G>
+template <int KC0, int KC1, bool TRACE, int G, int PIPE>
 __global__ void __launch_bounds__(128 * G)
 sgemm_dec_cluster2_kernel(const DecGemmArgs p0, const DecGemmArgs p1, const int tiles0) {
-  if ((int)blockIdx.x < tiles0) dec_cluster_body<KC0, TRACE, 8, G>(p0, (int)blockIdx.x);
-  else dec_cluster_body<KC1, TRACE, 8, G>(p1, (int)blockIdx.x - tiles0);
+  if ((int)blockIdx.x < tiles0) dec_cluster_body<KC0, TRACE, 8, G, PIPE>(p0, (int)blockIdx.x);
+  else dec_cluster_body<KC1, TRACE, 8, G, PIPE>(p1, (int)blockIdx.x - tiles0);
 }
 
 // One warp group (128 threads) per CTA.  The body is also written for G = 2 groups that split the CTA's K chunk once
 // more and are summed through shared memory; measured on a B200 that is slower (437.8 vs 429.1 ms per batch,
 // profiles/r02_call1_*): the multiply loop is bound by shared-memory bandwidth (8 LDS.128 per 64 FMAs with 4 x 4
 // register tiles), not by issue latency, so more warps only add the combine step.  For the same reason FFMA2 is not
-// faster than scalar FFMA here.
+// faster than scalar FFMA here.  (The staged loads of MT3_DEC_PIPE bit 0 are written for one group only.)
 constexpr int kDecGroups = 1;
 
-template <int KC0, int KC1, int G>
+// runtime MT3_DEC_PIPE bits -> the kernel instantiation
+#define MT3_DEC_PIPE_DISPATCH(pipe, CALL) \
+  switch ((pipe) & 3) {                   \
+    case 0: return CALL(0);               \
+    case 1: return CALL(1);               \
+    case 2: return CALL(2);               \
+    default: return CALL(3);              \
+  }
+
+template <int KC0, int KC1, int G, int PIPE>
 inline int launch_dec_gemm_cluster2_g(const DecGemmArgs& a0, const DecGemmArgs& a1, cudaStream_t s, bool pdl) {
-  constexpr size_t smem = dec_cluster_smem<(KC0 > KC1 ? KC0 : KC1), G>();
+  constexpr size_t smem = dec_cluster_smem<(KC0 > KC1 ? KC0 : KC1), G, PIPE>();
   static bool attr_done = false;
   if (!attr_done) {
-    MT3_CUDA_CHECK(cudaFuncSetAttribute(sgemm_dec_cluster2_kernel<KC0, KC1, false, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    MT3_CUDA_CHECK(cudaFuncSetAttribute(sgemm_dec_cluster2_kernel<KC0, KC1, true, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    MT3_CUDA_CHECK(cudaFuncSetAttribute(sgemm_dec_cluster2_kernel<KC0, KC1, false, G, PIPE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    MT3_CUDA_CHECK(cudaFuncSetAttribute(sgemm_dec_cluster2_kernel<KC0, KC1, true, G, PIPE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_done = true;
   }
   const int tiles0 = a0.N / kDecBN, tiles1 = a1.N / kDecBN;
   if (a0.trace)
-    MT3_CUDA_CHECK(launch_kernel_cluster(sgemm_dec_cluster2_kernel<KC0, KC1, true, G>, dim3(tiles0 + tiles1, 8), dim3(128 * G), smem, s,
+    MT3_CUDA_CHECK(launch_kernel_cluster(sgemm_dec_cluster2_kernel<KC0, KC1, true, G, PIPE>, dim3(tiles0 + tiles1, 8), dim3(128 * G), smem, s,
                                          pdl, 8u, a0, a1, tiles0));
   else
-    MT3_CUDA_CHECK(launch_kernel_cluster(sgemm_dec_cluster2_kernel<KC0, KC1, false, G>, dim3(tiles0 + tiles1, 8), dim3(128 * G), smem, s,
+    MT3_CUDA_CHECK(launch_kernel_cluster(sgemm_dec_cluster2_kernel<KC0, KC1, false, G, PIPE>, dim3(tiles0 + tiles1, 8), dim3(128 * G), smem, s,
                                          pdl, 8u, a0, a1, tiles0));
   MT3_LAUNCH_CHECK();
   return MT3_OK;
 }
 
 // the mt3 shapes: K = 384 (out-projection) and K = 384 + 512 (precomposed query block)
-inline int launch_dec_gemm_out_q(const DecGemmArgs& a0, const DecGemmArgs& a1, cudaStream_t s, bool pdl) {
+inline int launch_dec_gemm_out_q(const DecGemmArgs& a0, const DecGemmArgs& a1, cudaStream_t s, bool pdl, int pipe) {
   if (a0.M > kDecBM || a1.M > kDecBM || a0.K != 8 * 48 || a1.K != 8 * 112 || a0.N % kDecBN != 0 || a1.N % kDecBN != 0)
     return MT3_ERR_UNSUPPORTED;
-  return launch_dec_gemm_cluster2_g<48, 112, kDecGroups>(a0, a1, s, pdl);
+#define MT3_CALL(P) launch_dec_gemm_cluster2_g<48, 112, kDecGroups, P>(a0, a1, s, pdl)
+  MT3_DEC_PIPE_DISPATCH(pipe, MT3_CALL)
+#undef MT3_CALL
 }
 
-template <int KC, int S, int G>
+template <int KC, int S, int G, int PIPE>
 inline int launch_dec_gemm_cluster_kc(const DecGemmArgs& a, cudaStream_t s, bool pdl) {
-  constexpr size_t smem = dec_cluster_smem<KC, G>();
+  constexpr size_t smem = dec_cluster_smem<KC, G, PIPE>();
   static bool attr_done = false;
   if (!attr_done) {
-    MT3_CUDA_CHECK(cudaFuncSetAttribute(sgemm_dec_cluster_kernel<KC, false, S, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    MT3_CUDA_CHECK(cudaFuncSetAttribute(sgemm_dec_cluster_kernel<KC, true, S, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    MT3_CUDA_CHECK(cudaFuncSetAttribute(sgemm_dec_cluster_kernel<KC, false, S, G, PIPE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    MT3_CUDA_CHECK(cudaFuncSetAttribute(sgemm_dec_cluster_kernel<KC, true, S, G, PIPE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (S > 8) {
-      MT3_CUDA_CHECK(cudaFuncSetAttribute(sgemm_dec_cluster_kernel<KC, false, S, G>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-      MT3_CUDA_CHECK(cudaFuncSetAttribute(sgemm_dec_cluster_kernel<KC, true, S, G>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+      MT3_CUDA_CHECK(cudaFuncSetAttribute(sgemm_dec_cluster_kernel<KC, false, S, G, PIPE>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+      MT3_CUDA_CHECK(cudaFuncSetAttribute(sgemm_dec_cluster_kernel<KC, true, S, G, PIPE>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
     }
     attr_done = true;
   }
   if (a.trace)
-    MT3_CUDA_CHECK(launch_kernel_cluster(sgemm_dec_cluster_kernel<KC, true, S, G>, dim3(cdiv(a.N, kDecBN), S), dim3(128 * G), smem, s, pdl, (unsigned)S, a));
+    MT3_CUDA_CHECK(launch_kernel_cluster(sgemm_dec_cluster_kernel<KC, true, S, G, PIPE>, dim3(cdiv(a.N, kDecBN), S), dim3(128 * G), smem, s, pdl, (unsigned)S, a));
   else
-    MT3_CUDA_CHECK(launch_kernel_cluster(sgemm_dec_cluster_kernel<KC, false, S, G>, dim3(cdiv(a.N, kDecBN), S), dim3(128 * G), smem, s, pdl, (unsigned)S, a));
+    MT3_CUDA_CHECK(launch_kernel_cluster(sgemm_dec_cluster_kernel<KC, false, S, G, PIPE>, dim3(cdiv(a.N, kDecBN), S), dim3(128 * G), smem, s, pdl, (unsigned)S, a));
   MT3_LAUNCH_CHECK();
   return MT3_OK;
 }
 
+template <int KC, int S, int G>
+inline int launch_dec_gemm_cluster_p(const DecGemmArgs& a, cudaStream_t s, bool pdl, int pipe) {
+#define MT3_CALL(P) launch_dec_gemm_cluster_kc<KC, S, G, P>(a, s, pdl)
+  MT3_DEC_PIPE_DISPATCH(pipe, MT3_CALL)
+#undef MT3_CALL
+}
+
 template <int G>
-inline int launch_dec_gemm_cluster_g(const DecGemmArgs& a, cudaStream_t s, bool pdl) {
+inline int launch_dec_gemm_cluster_g(const DecGemmArgs& a, cudaStream_t s, bool pdl, int pipe) {
   // the long-K, narrow-N GEMM (MLP out: K = 1024, N = 512) has only N/32 x 8 = 128 CTAs at cluster size 8: a
   // cluster of 16 halves every CTA's K chunk and fills the machine
-  if ( a.K == 1024 && a.epi != EPI_GATED_GELU && a.N <= 512) return launch_dec_gemm_cluster_kc<64, 16, G>(a, s, pdl);
+  if ( a.K == 1024 && a.epi != EPI_GATED_GELU && a.N <= 512) return launch_dec_gemm_cluster_p<64, 16, G>(a, s, pdl, pipe);
   switch (a.K / 8) {
-    case 48: return launch_dec_gemm_cluster_kc<48, 8, G>(a, s, pdl);
-    case 64: return launch_dec_gemm_cluster_kc<64, 8, G>(a, s, pdl);
-    case 128: return launch_dec_gemm_cluster_kc<128, 8, G>(a, s, pdl);
+    case 48: return launch_dec_gemm_cluster_p<48, 8, G>(a, s, pdl, pipe);
+    case 64: return launch_dec_gemm_cluster_p<64, 8, G>(a, s, pdl, pipe);
+    case 128: return launch_dec_gemm_cluster_p<128, 8, G>(a, s, pdl, pipe);
     default: return MT3_ERR_UNSUPPORTED;
   }
 }
 
 // Returns MT3_ERR_UNSUPPORTED (without launching) when K does not split into 8 chunks of 48/64/128.
-inline int launch_dec_gemm_cluster(const DecGemmArgs& a, cudaStream_t s, bool pdl) {
+// pipe: MT3_DEC_PIPE bits (dec_cluster_body).
+inline int launch_dec_gemm_cluster(const DecGemmArgs& a, cudaStream_t s, bool pdl, int pipe) {
   if (a.M > kDecBM || a.N % 4 != 0 || a.lda % 4 != 0 || a.ldw % 4 != 0 || a.n_split % 4 != 0 || a.K % 8 != 0) return MT3_ERR_UNSUPPORTED;
-  return launch_dec_gemm_cluster_g<kDecGroups>(a, s, pdl);
+  return launch_dec_gemm_cluster_g<kDecGroups>(a, s, pdl, pipe);
 }
 
 inline int launch_dec_gemm(const DecGemmArgs& a, cudaStream_t s, bool pdl = false) {

@@ -98,6 +98,9 @@ struct Model {
   int pf_attn = 16;               // MT3_PF_ATTN=n: the decode-step attention kernels prefetch the n K/V tiles that follow their
                                   // shared-memory ring into L2 while they wait under the preceding GEMM (decode.cuh; value-neutral;
                                   // 0 = off: 449.6 -> 442.3 ms per batch at 16, profiles/r02_call63_ab_l2_prefetch.txt)
+  int dec_pipe = 3;               // MT3_DEC_PIPE bits of the cluster decode GEMM (decode.cuh dec_cluster_body): 1 = staged
+                                  // operand loads, 2 = exchange by bulk DSMEM copies, 0 = neither; bit-identical results
+                                  // (0 -> 3: 453.6 -> 428.8 ms per batch on a B200, profiles/r03_call3_bench_*)
   int kv_fmt = 0;                 // cfg.kv_cache_format: storage format of the self and cross K/V rows (kv_dest())
   int kv_row = 256;               // bytes per K/V row of 64 elements
   // debug timeline (mt3_debug_trace_step): while `tracing` is set every decode GEMM / attention launch gets a slot
@@ -419,7 +422,7 @@ static int dec_gemm(Model* m, const float* A, int lda, const float* W, int N, in
     a.counters = m->dcounters;
     a.trace = trace_slot(m, K == m->F ? "gemm_mlp_out" : (N == 2 * m->F ? "gemm_mlp_in" : (kv ? "gemm_qkv_append" : (N == m->V ? "gemm_logits" : (K == m->Q ? "gemm_attn_out" : "gemm_cross_q")))));
     int rc = MT3_ERR_UNSUPPORTED;
-    if (m->dec_cluster) rc = launch_dec_gemm_cluster(a, s, m->pdl_gemm);
+    if (m->dec_cluster) rc = launch_dec_gemm_cluster(a, s, m->pdl_gemm, m->dec_pipe);
     if (rc == MT3_ERR_UNSUPPORTED) rc = launch_dec_gemm(a, s, m->pdl_gemm);   // shapes the cluster kernel does not tile
     MT3_TRY(rc);
   }
@@ -478,7 +481,7 @@ static int dec_gemm_out_q(Model* m, const DecLayer& w, const float* y_in, float*
   a1.eps = 1e-6f; a1.epi = EPI_STORE; a1.C = m->dq + r0 * Q; a1.ldc = Q; a1.n_split = Q;
   a1.R = a1.C; a1.ldr = Q;
   a1.trace = a0.trace;
-  return launch_dec_gemm_out_q(a0, a1, s, m->pdl_gemm);
+  return launch_dec_gemm_out_q(a0, a1, s, m->pdl_gemm, m->dec_pipe);
 }
 
 // The residual stream of one step (ping-pongs between m->dy and m->dy2 across fused launches).
@@ -772,6 +775,8 @@ extern "C" int mt3_model_create(const mt3_model_config* cfg, const float* weight
     m->tc_attn_ok = !(e_attn && e_attn[0] == '0');
     const char* e_pfa = getenv("MT3_PF_ATTN");
     if (e_pfa) m->pf_attn = std::max(0, atoi(e_pfa));
+    const char* e_pipe = getenv("MT3_DEC_PIPE");
+    if (e_pipe) m->dec_pipe = atoi(e_pipe) & 3;
   }
   m->kv_fmt = cfg->kv_cache_format;
   m->kv_row = kv_row_bytes(m->kv_fmt);

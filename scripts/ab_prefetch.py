@@ -20,7 +20,7 @@ import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
-KNOBS = ("MT3_PF_ATTN", "MT3_PDL", "MT3_DEC_FUSE", "MT3_DEC_CLUSTER")
+KNOBS = ("MT3_PF_ATTN", "MT3_PDL", "MT3_DEC_FUSE", "MT3_DEC_CLUSTER", "MT3_DEC_PIPE")
 
 DEFAULT = ";".join(["off:MT3_PF_ATTN=0", "attn4:MT3_PF_ATTN=4", "attn8:MT3_PF_ATTN=8", "default:", "attn32:MT3_PF_ATTN=32",
                     "attn64:MT3_PF_ATTN=64", "off2:MT3_PF_ATTN=0"])

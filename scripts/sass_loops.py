@@ -2,7 +2,7 @@
 opcodes between its target and the branch are counted.  Used for the static side of DESIGN.md's roofline arguments (what
 one trip of the decode GEMM's multiply loop issues, how many UBLKCP / UBLKPF the attention producer holds, ...).
 
-    python scripts/sass_loops.py 'sgemm_dec_cluster_kernel<64, false, 8, 1>' [more kernel-name substrings ...]
+    python scripts/sass_loops.py 'sgemm_dec_cluster_kernel<64, false, 8, 1, 3>' [more kernel-name substrings ...]
 """
 import collections
 import os
@@ -41,7 +41,7 @@ def loops(ins):
 
 
 def main():
-    pats = sys.argv[1:] or ["sgemm_dec_cluster_kernel<64, false, 8, 1>"]
+    pats = sys.argv[1:] or ["sgemm_dec_cluster_kernel<64, false, 8, 1, 3>"]
     ks = kernels()
     for name, ins in ks.items():
         if not any(p in name for p in pats):
